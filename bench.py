@@ -32,6 +32,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -172,6 +173,24 @@ def cpu_reference(n_envs: int, seconds: float, warmup: int, seed: int, nthreads:
     return n_envs * steps / dt, nthreads, dt, steps
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """arrays: name -> [num_envs, ...] numpy array.  Float arrays keep their width, integer flags become float32.  Above
+    DUMP_LIMIT_BYTES the same fixed, seeded sample of environment rows is taken from every array."""
+    import numpy as np
+    arrays = {k: v.astype(v.dtype if v.dtype in (np.float32, np.float64) else np.float32) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(v.nbytes // n for v in arrays.values())
+    if n * row_bytes > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -190,7 +209,15 @@ def main():
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--workload", default="jvrc_walk", choices=sorted(WORKLOADS),
                     help="jvrc_walk: the configuration BASELINE.json's metric is quoted on (default); jvrc_step: configs[2]; h1: configs[3]; jvrc_walk_terrain: configs[4] (extension)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (obs, reward, done, ended of rank 0's "
+                         "environments) to DIR/<name>.npy as float32 / float64, at most 64 MB in all (a fixed, seeded sample of "
+                         "environments beyond that), so that two builds can be compared output for output on the same inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm runs for a wall-time budget, not a fixed number of steps)")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -310,6 +337,9 @@ def main():
     total_ms = sum(step_ms)
     launches = K          # one lhw_sim_step launch per timed step (lhw_launch_count also counts the warm-up)
     assert _lib.lib().lhw_launch_count() - launches0 == K + W + PREROLL
+    # env.step returns its own output buffers: until the next step they hold what the last timed step computed
+    last_outputs = {name: t.cpu().numpy() for name, t in zip(("obs", "reward", "done", "ended"),
+                                                            (env.obs, env.reward, env.done, env.ended))} if args.dump_outputs else None
     # ---- e2e: pinned host actions in, pinned host obs/reward/done out, every step
     h_acts = torch.empty(K, n, A, dtype=env.dtype).pin_memory()
     h_acts.copy_(acts.cpu())     # the policy regime's e2e leg plays the same exploration noise open loop (the host owns the actions)
@@ -451,6 +481,8 @@ def main():
             out["cpu_baseline"] = {"value": sps, "unit": UNIT, "cores": threads, "kind": "port",
                                    "sample": f"{n} envs (the GPU arm's batch) x {nst} control steps ({dt:.1f} s) after 2 warm-up steps, same "
                                              "action distribution; oracle/ C port with OpenMP (reference Ray+MuJoCo path not installable here)"}
+        if last_outputs is not None:
+            dump_outputs(args.dump_outputs, last_outputs)
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
@@ -475,6 +507,7 @@ def bench_train_iter(args, wl, rank, world, local_rank, barrier):
     spec.loader.exec_module(rx)
     flags = {f[2:].replace("-", "_"): (False if kw.get("action") == "store_true" else kw.get("default")) for f, kw in rx.TRAIN_FLAGS}
     os.environ.setdefault("LHW_TENSORBOARD", "0")
+    logdir = tempfile.TemporaryDirectory(prefix="lhw_bench_train_")     # the trainer's run directory: never in the tree
     dev = torch.device("cuda", local_rank)
     n, T, iters = args.envs, 400, 2
     out = {"definition": "samples / (sampling + optimisation time) as rl/algos/ppo.py:587-595, whole job, max over ranks of the wall "
@@ -491,7 +524,7 @@ def bench_train_iter(args, wl, rank, world, local_rank, barrier):
         env_fn = base if not hasattr(r, "mirrored_obs") else partial(SymmetricEnv, base, mirrored_obs=r.mirrored_obs,
                                                                      mirrored_act=r.mirrored_acts, clock_inds=r.clock_inds)
         a = SimpleNamespace(**flags)
-        a.num_procs, a.logdir, a.seed, a.eval_freq, a.eval_at_start, a.steps_per_env = n, "/tmp/lhw_bench_train", args.seed, 10 ** 9, False, T
+        a.num_procs, a.logdir, a.seed, a.eval_freq, a.eval_at_start, a.steps_per_env = n, logdir.name, args.seed, 10 ** 9, False, T
         a.env, a.precision = wl["model"], prec
         ppo = PPO(env_fn, a, seed=args.seed)
         ppo.train(None, 1, verbose=False)
@@ -553,6 +586,7 @@ def bench_train_iter(args, wl, rank, world, local_rank, barrier):
                   "torch.distributed NCCL all_reduce + lhw_grad_sumsq / lhw_clip_adam_dev per network (7 launches)")
     out["exchange_us"] = ex
     comm.close()
+    logdir.cleanup()
     return out
 
 

@@ -50,17 +50,16 @@ def test_product_never_imports_the_oracle():
 
 def test_run_experiment_keeps_the_reference_flags():
     """run_experiment.py (repo root) accepts every flag of the reference's entry point (run_experiment.py:152-260).  The flag
-    list below was read off the reference; where the reference checkout is present (this container, not the GPU box) it is
-    re-derived from the file itself."""
+    list below was read off the reference; where LHW_REFERENCE names a checkout of it, it is re-derived from the file itself."""
     src = open(os.path.join(ROOT, "run_experiment.py")).read()
     ours = set(re.findall(r"\(\"(--[a-z-]+)\",", src))
     ref_flags = {"--env", "--logdir", "--input-norm-steps", "--n-itr", "--lr", "--eps", "--gamma", "--lam", "--std-dev",
                  "--learn-std", "--entropy-coeff", "--clip", "--minibatch-size", "--epochs", "--num-procs", "--max-grad-norm",
                  "--max-traj-len", "--no-mirror", "--mirror-coeff", "--eval-freq", "--continued", "--recurrent", "--imitate",
                  "--imitate-coeff", "--yaml", "--device", "--seed", "--path", "--out-dir", "--ep-len"}
-    ref_file = "/root/reference/run_experiment.py"
-    if os.path.exists(ref_file):
-        assert set(re.findall(r"\"(--[a-z-]+)\"", open(ref_file).read())) == ref_flags
+    ref = os.environ.get("LHW_REFERENCE")
+    if ref:
+        assert set(re.findall(r"\"(--[a-z-]+)\"", open(os.path.join(ref, "run_experiment.py")).read())) == ref_flags
     assert ref_flags <= ours, ref_flags - ours
 
 

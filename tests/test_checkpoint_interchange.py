@@ -5,7 +5,7 @@ rl/utils/checkpointer.py:36-83, loaded back at run_experiment.py:274-277 and rl/
                             (tools/gen_golden_ckpt.py); they load here with no reference on the path, give the recorded
                             outputs, and PPO.load_pretrained takes their weights / normalisation but not their stds.
   this build -> reference   a pair written by PPO.save's exporter is unpickled in a fresh interpreter that has ONLY the
-                            reference on its path (this container; skipped on the GPU box where /root/reference is absent).
+                            reference on its path (LHW_REFERENCE names the checkout; skipped without one).
 """
 import io
 import json
@@ -19,7 +19,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = os.path.join(HERE, "golden")
-REF = "/root/reference"
+REF = os.environ.get("LHW_REFERENCE", "")     # a checkout of rohanpsingh/LearningHumanoidWalking, if one is at hand
 
 
 def test_reference_checkpoint_loads_here_and_gives_the_recorded_outputs():
@@ -96,7 +96,7 @@ def test_exported_files_name_the_reference_classes_and_hold_only_their_own_param
     assert torch.equal(back(x), actor(x))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="needs the reference checkout (this container only)")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs LHW_REFERENCE: a checkout of the upstream project")
 def test_a_reference_checkout_unpickles_our_files_with_its_own_classes(tmp_path):
     actor, critic, pa, pc = _export_pair(tmp_path)
     x = torch.randn(4, 37)

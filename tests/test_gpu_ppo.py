@@ -3,6 +3,7 @@ against oracle/ppo_oracle.py (pinned to the reference's PPOBuffer by tests/golde
 DeviceRolloutWorker / PPO host classes against the reference's behavioural contract (tests/test_training.py)."""
 import json
 import os
+import tempfile
 from types import SimpleNamespace
 
 import numpy as np
@@ -127,10 +128,14 @@ def test_fused_clip_adam_matches_torch_clip_grad_norm_and_adam():
         assert np.abs(opt_a.flat.double().cpu().numpy() - p).max() < 2e-6
 
 
+# checkpoints of the training runs below go to a private directory (a fixed /tmp path may belong to another user), removed at exit
+_LOGDIR = tempfile.TemporaryDirectory(prefix="lhw_test_logs_")
+
+
 def _args(**kw):
     d = dict(gamma=0.99, lam=0.95, lr=3e-4, eps=1e-5, entropy_coeff=0.0, clip=0.2, minibatch_size=256, epochs=1,
              max_traj_len=50, num_procs=64, max_grad_norm=0.05, mirror_coeff=0.4, eval_freq=100, recurrent=False,
-             imitate_coeff=0.0, std_dev=0.223, learn_std=False, logdir="/tmp/lhw_test_logs", steps_per_env=20)
+             imitate_coeff=0.0, std_dev=0.223, learn_std=False, logdir=_LOGDIR.name, steps_per_env=20)
     d.update(kw)
     return SimpleNamespace(**d)
 

@@ -112,7 +112,8 @@ def test_model_constants():
     assert abs(m["total_mass"] * 9.8 * 0.5 - 305.76) < 1e-9
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(os.environ.get("LHW_REFERENCE", "")),
+                    reason="needs LHW_REFERENCE: a checkout of the upstream project")
 def test_compiled_model_is_reproducible_from_reference():
     import sys
     sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(__file__)), "tools"))

@@ -31,7 +31,11 @@ def test_committed_evaluation_bounds_the_proxy_error():
         assert all(legs[a] != legs[b] for a, b in sc["pairs"])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models/jvrc_mj_description/meshes/convex"), reason="needs the reference's STL hulls")
+REF = os.environ.get("LHW_REFERENCE", "")     # a checkout of rohanpsingh/LearningHumanoidWalking, if one is at hand
+
+
+@pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, "models/jvrc_mj_description/meshes/convex")),
+                    reason="needs LHW_REFERENCE: a checkout of the upstream project (its STL hulls)")
 def test_spot_check_against_the_hulls():
     import sys
     sys.path.insert(0, ROOT)

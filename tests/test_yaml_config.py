@@ -6,7 +6,7 @@ import os
 import numpy as np
 import pytest
 
-REF = "/root/reference"
+REF = os.environ.get("LHW_REFERENCE", "")     # a checkout of rohanpsingh/LearningHumanoidWalking, if one is at hand
 
 
 def _write(tmp_path, text):
@@ -63,7 +63,7 @@ def test_yaml_rejects_what_it_cannot_honour(tmp_path):
     assert m["cfg"]["perturbation"]["force_magnitude"] == 30 and m["cfg"]["perturbation"]["torque_magnitude"] == 2
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="needs the reference checkout (this container only)")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs LHW_REFERENCE: a checkout of the upstream project")
 @pytest.mark.parametrize("model,rel", [("jvrc_walk", "envs/jvrc/configs/base.yaml"), ("jvrc_step", "envs/jvrc/configs/base.yaml"),
                                        ("h1", "envs/h1/configs/base.yaml")])
 def test_the_references_own_yaml_is_the_compiled_configuration(model, rel):
